@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the warp / filter engine (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch B]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch B] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one ``warp_perspective`` call on a synthetic B x 3 x 1080 x 1920 fp32 batch
@@ -19,6 +19,8 @@ One JSON line on stdout (rank 0):
             bounded sample (rank 0, N=1 only)
 ``--impl reference`` times that CPU port alone (the reference is pure Python and cannot travel to
 the GPU box; the port issues the same ATen calls: oracle/kornia_restated.py).
+``--dump-outputs DIR`` writes what the last timed step returned as DIR/<name>.npy (see dump_outputs); the inputs
+are generated from fixed seeds, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -80,6 +82,34 @@ def make_homographies_hw(B: int, seed: int, Hh: int, Ww: int) -> torch.Tensor:
 
 def make_homographies(B: int, seed: int) -> torch.Tensor:
     return make_homographies_hw(B, seed, H_IMG, W_IMG)
+
+
+# ------------------------------------------------------------------------------------------ outputs
+DUMP_BYTES = 60 * 10**6  # array data written by --dump-outputs; with the .npy headers the files stay under 64 MB
+
+
+def dump_outputs(directory: str, arrays: dict) -> None:
+    """Write what the timed path returned as ``directory/<name>.npy`` (float64 tensors as float64, all others as float32),
+    so that two builds run with the same arguments can be compared output for output.  Arrays are taken smallest first and
+    each may use an equal share of what is left of DUMP_BYTES: one that fits is written whole, a larger one as the elements
+    at a fixed set of flat indices (drawn with seed 0, sorted; the same for every run with the same shape), flattened."""
+    import numpy as np
+
+    os.makedirs(directory, exist_ok=True)
+    left, todo = DUMP_BYTES, sorted(arrays.items(), key=lambda kv: kv[1].numel())
+    for i, (name, t) in enumerate(todo):
+        t = t.detach()
+        t = t.double() if t.dtype == torch.float64 else t.float()
+        share = left // (len(todo) - i)
+        if t.numel() * t.element_size() <= share:
+            a, note = t.cpu().numpy(), "whole"
+        else:
+            k = share // t.element_size()
+            idx = torch.randint(t.numel(), (k,), generator=torch.Generator().manual_seed(0)).unique()
+            a, note = t.reshape(-1)[idx.to(t.device)].cpu().numpy(), f"{idx.numel()} of {t.numel()} elements at seeded indices"
+        np.save(os.path.join(directory, name + ".npy"), a)
+        left -= a.nbytes
+        print(f"bench.py: wrote {name}.npy {tuple(t.shape)} {a.dtype} ({note})", file=sys.stderr)
 
 
 # ------------------------------------------------------------------------------------------ clocks
@@ -472,6 +502,8 @@ def run_ours(args) -> None:
     total_ms = t0.elapsed_time(t1)
     kern_ms = [s.elapsed_time(e) for (_, s, e) in timed_events]
     checksum = float(out[0, :, ::97, ::89].sum())  # touch the result
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"out": out})
     del out
     if dist is not None:
         t = torch.tensor([total_ms], device=dev)
@@ -606,12 +638,15 @@ def run_extra(args) -> None:
     with ClockSampler(dev.index or 0) as clk:
         t0.record()
         for _ in range(args.steps):
-            step()
+            res = step()
         t1.record()
         torch.cuda.synchronize(dev)
         timed_events, _ops.kernel_events = (_ops.kernel_events or []), None
         launches = _ops.launch_count - launches0
         clk.hold_load(step, lambda: torch.cuda.synchronize(dev))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dict(zip(("grad_src", "grad_M"), res)) if args.workload == "warp_bwd" else {"out": res})
+    del res
     ms = t0.elapsed_time(t1) / args.steps
     kern = [s.elapsed_time(e) for (tg, s, e) in timed_events if tg == tag]
     k_ms = statistics.mean(kern) if kern else None
@@ -865,7 +900,13 @@ def main() -> None:
     ap.add_argument("--workload", choices=["warp", "blur", "warp_bwd", "ingest", "small", "scatter_gather"], default="warp",
                     help="warp = the headline (BASELINE.json configs[1]); blur / warp_bwd = configs[2] / configs[3]; ingest = the uint8 wire-format warp "
                          "(SURVEY 8f row 4, not a BASELINE config); single GPU")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last step returned as DIR/<name>.npy "
+                    "(float32 / float64, under 64 MB in all: a larger output as a fixed, seeded sample); warp, blur, warp_bwd and ingest")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.workload in ("small", "scatter_gather")):
+        ap.error("--dump-outputs covers the warp, blur, warp_bwd and ingest workloads of --impl ours")
     if args.impl == "reference":
         run_reference(args)
     elif args.workload == "small":

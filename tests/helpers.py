@@ -1,4 +1,9 @@
 """Shared helpers for the parity tests: dispatch a golden case onto an implementation module."""
+import json
+import os
+import sys
+import types
+
 import torch
 
 
@@ -79,3 +84,35 @@ def family_grads(impl, op, kwargs, ins, outs, device=None, dtype=None):
     res = {"out": out.detach()}
     res.update({f"grad_{k}": g for k, g in zip(wrt, grads)})
     return res
+
+
+def reference_package(monkeypatch):
+    """The reference's ``kornia`` package as tests/golden/install.json records it (make_golden_install.py): every module,
+    its attributes that name other modules of the package, and the functions ``kornia_b200.install()`` rebinds, bound
+    under the same names in the same modules as in the reference, one stand-in object per function.  The modules are in
+    ``sys.modules`` until the test ends.  Returns the top-level package and the recorded (module name, function name)
+    bindings."""
+    with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "install.json")) as f:
+        rec = json.load(f)
+
+    def stand_in(name):
+        def fn(*args, **kwargs):
+            raise AssertionError(f"the reference's {name} was called")
+
+        fn.__name__ = fn.__qualname__ = name
+        return fn
+
+    originals = {name: stand_in(name) for name in rec["defining"]}
+    mods = {name: types.ModuleType(name) for name in rec["modules"]}
+    for name, m in mods.items():
+        parent, _, leaf = name.rpartition(".")
+        if parent:
+            setattr(mods[parent], leaf, m)
+        monkeypatch.setitem(sys.modules, name, m)
+    # after the submodule attributes: ``from .sobel import sobel`` leaves the function, not the module, in kornia.filters
+    for name, r in rec["modules"].items():
+        for attr, target in r["aliases"].items():
+            setattr(mods[name], attr, mods[target])
+        for fn in r["binds"]:
+            setattr(mods[name], fn, originals[fn])
+    return mods["kornia"], [(m, fn) for m, r in rec["modules"].items() for fn in r["binds"]]

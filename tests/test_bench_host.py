@@ -19,3 +19,22 @@ def test_ring_is_whole_chunks_within_a_third_of_the_ranks_share():
 
 def test_small_batches_are_never_cut():
     assert bench.host_ring_samples(8, 16, available_bytes=GIB, local_ranks=8) == 8
+
+
+def test_dump_outputs_fits_the_budget_and_samples_the_same_elements(tmp_path, monkeypatch):
+    import numpy as np
+    import torch
+
+    monkeypatch.setattr(bench, "DUMP_BYTES", 4000)
+    big = torch.arange(10_000, dtype=torch.float32).reshape(10, 1000)
+    small = torch.arange(9, dtype=torch.float64).reshape(3, 3)
+    half = torch.ones(4, dtype=torch.float16)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), {"big": big, "small": small, "half": half})
+    a = {n: np.load(tmp_path / "a" / f"{n}.npy") for n in ("big", "small", "half")}
+    assert a["small"].dtype == np.float64 and np.array_equal(a["small"], small.numpy())  # fits: written whole
+    assert a["half"].dtype == np.float32 and a["half"].shape == (4,)
+    assert a["big"].dtype == np.float32 and a["big"].ndim == 1 and 0 < a["big"].size < big.numel()
+    assert np.all(np.diff(a["big"]) > 0)  # the elements of sorted, distinct flat indices
+    assert sum(x.nbytes for x in a.values()) <= 4000
+    assert np.array_equal(a["big"], np.load(tmp_path / "b" / "big.npy"))

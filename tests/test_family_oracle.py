@@ -3,14 +3,14 @@ restatement against the vectors recorded from the reference (tests/golden/family
 logic of the product wrappers (signatures, tap generators, matrix builders: pure torch, runs on
 CPU) and ``install()``."""
 import inspect
-import os
+import sys
 
 import pytest
 import torch
 
 import kornia_b200 as K
 from conftest import golden
-from helpers import family_grads, rel_l2, run_family_case
+from helpers import family_grads, reference_package, rel_l2, run_family_case
 from oracle import kornia_restated as R
 
 FAM = golden("family")
@@ -144,44 +144,43 @@ def test_module_forms():
     assert KF.UnsharpMask((3, 3), (1.0, 1.0)).border_type == "reflect"
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/kornia"), reason="needs the reference checkout (build container only)")
-def test_install_rebinds_every_importer_of_the_reference():
-    import sys
-    import tempfile
+def test_install_rebinds_every_importer_of_the_reference(monkeypatch):
+    """On the reference's import graph (recorded in tests/golden/install.json): every module that holds one of the
+    rebound functions gets the product's, and ``uninstall()`` puts the reference's back."""
+    kornia, bindings = reference_package(monkeypatch)
+    aug_persp = sys.modules["kornia.augmentation._2d.geometric.perspective"]
+    aug_blur = sys.modules["kornia.augmentation._2d.intensity.gaussian_blur"]
+    affwarp = sys.modules["kornia.geometry.transform.affwarp"]
+    crop2d = sys.modules["kornia.geometry.transform.crop2d"]
+    unsharp = sys.modules["kornia.filters.unsharp"]
+    ours = {"warp_perspective": K.warp_perspective, "warp_affine": K.warp_affine, "remap": K.remap, "filter2d": K.filter2d,
+            "filter2d_separable": K.filter2d_separable, "gaussian_blur2d": K.gaussian_blur2d,
+            "get_perspective_transform": K.geometry.transform.get_perspective_transform, "spatial_gradient": K.filters.spatial_gradient,
+            "sobel": K.filters.sobel, "ssim": K.metrics.ssim}
+    before = {(m, name): getattr(sys.modules[m], name) for m, name in bindings}
 
-    stub = tempfile.mkdtemp(prefix="kornia_rs_stub_")
-    open(os.path.join(stub, "kornia_rs.py"), "w").close()
-    sys.path[:0] = [stub, "/root/reference"]
+    orig = kornia.geometry.transform.imgwarp.warp_perspective
+    K.install(kornia)
     try:
-        import kornia
-        import kornia.augmentation._2d.geometric.perspective as aug_persp
-        import kornia.augmentation._2d.intensity.gaussian_blur as aug_blur
-        import kornia.geometry.transform.affwarp as affwarp
-        import kornia.geometry.transform.crop2d as crop2d
-        import kornia.filters.unsharp as unsharp
-
-        orig = kornia.geometry.transform.imgwarp.warp_perspective
-        K.install(kornia)
-        try:
-            assert kornia.geometry.transform.warp_perspective is K.warp_perspective
-            assert kornia.geometry.warp_affine is K.warp_affine
-            assert kornia.filters.gaussian_blur2d is K.gaussian_blur2d
-            assert aug_persp.warp_perspective is K.warp_perspective      # RandomPerspective.apply_transform
-            assert affwarp.warp_affine is K.warp_affine                  # affine / rotate / translate / scale / shear
-            assert crop2d.warp_perspective is K.warp_perspective and crop2d.warp_affine is K.warp_affine
-            assert unsharp.gaussian_blur2d is K.gaussian_blur2d
-            assert aug_blur.gaussian_blur2d is K.gaussian_blur2d                 # captured by RandomGaussianBlur.__init__
-            assert aug_persp.get_perspective_transform is K.geometry.transform.get_perspective_transform
-            assert kornia.filters.sobel is K.filters.sobel and kornia.filters.spatial_gradient is K.filters.spatial_gradient
-            assert kornia.metrics.ssim is K.metrics.ssim and kornia.losses.ssim.metrics.ssim is K.metrics.ssim
-            K.install(kornia)  # idempotent: the originals are remembered once
-        finally:
-            K.uninstall()
-        assert kornia.geometry.transform.warp_perspective is orig and aug_persp.warp_perspective is orig
-        assert kornia.metrics.ssim is not K.metrics.ssim and callable(kornia.filters.sobel)
+        assert kornia.geometry.transform.warp_perspective is K.warp_perspective
+        assert kornia.geometry.warp_affine is K.warp_affine
+        assert kornia.filters.gaussian_blur2d is K.gaussian_blur2d
+        assert aug_persp.warp_perspective is K.warp_perspective      # RandomPerspective.apply_transform
+        assert affwarp.warp_affine is K.warp_affine                  # affine / rotate / translate / scale / shear
+        assert crop2d.warp_perspective is K.warp_perspective and crop2d.warp_affine is K.warp_affine
+        assert unsharp.gaussian_blur2d is K.gaussian_blur2d
+        assert aug_blur.gaussian_blur2d is K.gaussian_blur2d                 # captured by RandomGaussianBlur.__init__
+        assert aug_persp.get_perspective_transform is K.geometry.transform.get_perspective_transform
+        assert kornia.filters.sobel is K.filters.sobel and kornia.filters.spatial_gradient is K.filters.spatial_gradient
+        assert kornia.metrics.ssim is K.metrics.ssim and kornia.losses.ssim.metrics.ssim is K.metrics.ssim
+        missed = [(m, name) for m, name in bindings if getattr(sys.modules[m], name) is not ours[name]]
+        assert not missed, missed
+        K.install(kornia)  # idempotent: the originals are remembered once
     finally:
-        sys.path.remove(stub)
-        sys.path.remove("/root/reference")
+        K.uninstall()
+    assert kornia.geometry.transform.warp_perspective is orig and aug_persp.warp_perspective is orig
+    assert kornia.metrics.ssim is not K.metrics.ssim and callable(kornia.filters.sobel)
+    assert all(getattr(sys.modules[m], name) is before[m, name] for m, name in bindings)
 
 
 def test_fused_unsharp_request_host_logic():

@@ -2,7 +2,6 @@
 against the vectors recorded from the reference (tests/golden/wider.npz), the product wrappers' host logic with the
 core functions swapped for the oracle, the signatures and the error behaviour."""
 import inspect
-import os
 from importlib import import_module
 
 import pytest
@@ -10,7 +9,7 @@ import torch
 
 import kornia_b200 as K
 from conftest import golden
-from helpers import family_grads, rel_l2, run_family_case
+from helpers import family_grads, reference_package, rel_l2, run_family_case
 from oracle import kornia_restated as R
 
 WID = golden("wider")
@@ -152,31 +151,20 @@ def test_tilt_projection_matches_oracle():
     assert KC.tilt_projection(torch.tensor(0.1), torch.tensor(0.2)).shape == (3, 3)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/kornia"), reason="needs the reference checkout (build container only)")
-def test_install_reaches_the_new_callers():
+def test_install_reaches_the_new_callers(monkeypatch):
     """install() rebinds filter2d / gaussian_blur2d / remap inside the reference's pyramid, affwarp and undistort modules,
-    so the reference's own pyrdown / resize(antialias) / undistort_image run on the CUDA kernels unmodified."""
-    import sys
-    import tempfile
-
-    stub = tempfile.mkdtemp(prefix="kornia_rs_stub_")
-    open(os.path.join(stub, "kornia_rs.py"), "w").close()
-    sys.path[:0] = [stub, "/root/reference"]
+    so the reference's own pyrdown / resize(antialias) / undistort_image run on the CUDA kernels unmodified (on the
+    reference's import graph recorded in tests/golden/install.json)."""
+    kornia, _ = reference_package(monkeypatch)
+    pyr = import_module("kornia.geometry.transform.pyramid")
+    aff = import_module("kornia.geometry.transform.affwarp")
+    und = import_module("kornia.geometry.calibration.undistort")
+    K.install(kornia)
     try:
-        import kornia
-
-        pyr = import_module("kornia.geometry.transform.pyramid")
-        aff = import_module("kornia.geometry.transform.affwarp")
-        und = import_module("kornia.geometry.calibration.undistort")
-        K.install(kornia)
-        try:
-            assert pyr.filter2d is K.filter2d and aff.gaussian_blur2d is K.gaussian_blur2d and und.remap is K.remap
-        finally:
-            K.uninstall()
-        assert pyr.filter2d is not K.filter2d
+        assert pyr.filter2d is K.filter2d and aff.gaussian_blur2d is K.gaussian_blur2d and und.remap is K.remap
     finally:
-        sys.path.remove(stub)
-        sys.path.remove("/root/reference")
+        K.uninstall()
+    assert pyr.filter2d is not K.filter2d
 
 
 def test_lens_packing_and_kernel_op_order():
